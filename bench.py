@@ -10,6 +10,7 @@ of the named architecture (no checkpoints offline).
 
   python bench.py --gpus N --steps K --warmup W            # our sm_100a path (one rank per GPU under torchrun)
   python bench.py --impl reference --steps K --warmup W    # the reference algorithm (oracle port) on the host cores
+  python bench.py --steps K --dump-outputs DIR             # also writes the last timed step's token ids to DIR/tokens.npy
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for the definitions of value / e2e / roofline.
 """
@@ -210,16 +211,18 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """Returns (ms, tokens, output of the last step)."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         n_tok = 0
         for _ in range(steps):
-            n_tok += int(fn().numel())
+            out = fn()
+            n_tok += int(out.numel())
         e1.record()
         barrier()
         ms, n_tok, _ = aggregate_throughput(e0.elapsed_time(e1), n_tok, dev)  # max over ranks; tokens all-gathered
-        return ms, n_tok
+        return ms, n_tok, out
 
     for _ in range(max(args.warmup, 3)):
         step_device()
@@ -227,12 +230,17 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     ops.LAUNCHES = 0
-    ms, n_tok = timed(step_device, args.steps)
+    ms, n_tok, last_ids = timed(step_device, args.steps)
     launches = ops.LAUNCHES
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # token ids [1, NEW_TOKENS] of the last timed step; float64 holds every int64 id below 2^53 exactly
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "tokens.npy"), last_ids.cpu().numpy().astype(np.float64))
     for _ in range(2):
         step_e2e()
-    ms_e2e, n_tok_e2e = timed(step_e2e, args.steps)
+    ms_e2e, n_tok_e2e, _ = timed(step_e2e, args.steps)
 
     # ---- the mode the reference's driver actually runs (eval_spatial.py:223-237): an EOS id plus KeywordsStoppingCriteria,
     #      inspected after every token.  Stop checks are asynchronous in our decoder (llama_decoder._decode_loop), so this
@@ -258,14 +266,14 @@ def run_ours(args):
                              masks=[h_msk.to(dev, non_blocking=True)], eos_token_id=cfg.llama.vocab_size - 3, stopping_criteria=[crit], **gen_kw)
         return out.cpu()
     step_stop()
-    ms_stop, n_tok_stop = timed(step_stop, args.steps)
+    ms_stop, n_tok_stop, _ = timed(step_stop, args.steps)
 
     # ---- TTFT (2 tower passes + refinement + pooling + projector + splice + Llama prefill + first token): the
     #      "prefill TFLOPS vs roofline" half of BASELINE.json's metric, algorithmic FLOPs of SURVEY.md §8d
     def step_ttft():
         return model.generate(d_ids, images=d_img, depths=d_dep, masks=[d_msk], do_sample=False, max_new_tokens=1)
     step_ttft()
-    ms_ttft, _ = timed(step_ttft, args.steps)
+    ms_ttft, _, _ = timed(step_ttft, args.steps)
     ttft_ms = ms_ttft / args.steps
 
     # ---- per-kernel roofline of the dominant kernel, timed live with CUDA events: the gate/up GEMV
@@ -315,7 +323,7 @@ def run_ours(args):
         for _ in range(2):
             step_c3()
         l0 = ops.LAUNCHES
-        ms_c3, n_c3 = timed(step_c3, args.steps)
+        ms_c3, n_c3, _ = timed(step_c3, args.steps)
         c3_launches = (ops.LAUNCHES - l0) // args.steps
         c3_ms = ms_c3 / args.steps
         c3_flops = C3_BATCH * nums["flops_ttft"]
@@ -515,7 +523,14 @@ def main():
     ap.add_argument("--no-c3", action="store_true", help="skip the batch-32 prefill-only measurement (config c3)")
     ap.add_argument("--dtype", default="bf16", choices=["bf16", "fp16"],
                     help="compute dtype: bf16 (how the reference's eval_spatial.py runs the model; the graded default) or fp16 (the loader default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the token ids rank 0's last timed step returned to DIR/tokens.npy (float64); "
+                         "inputs and weights are seeded, so runs with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:
@@ -525,6 +540,8 @@ def main():
             cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",
                    "--master-addr", "127.0.0.1", "--master-port", "29511", os.path.abspath(__file__), "--gpus", str(args.gpus),
                    "--steps", str(args.steps), "--warmup", str(args.warmup), "--dtype", args.dtype]
+            if args.dump_outputs:
+                cmd += ["--dump-outputs", os.path.abspath(args.dump_outputs)]
             sys.exit(subprocess.call(cmd))
         run_ours(args)
 
