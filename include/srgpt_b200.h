@@ -157,6 +157,22 @@ int srgpt_rope_kv_append_bf16(void* qkv, int rows, int n_heads, int n_kv_heads, 
 int srgpt_rope_kv_append_varlen_bf16(void* qkv, int rows, int n_heads, int n_kv_heads, int head_dim, const void* cos_tab,
                                      const void* sin_tab, const int* start_pos, void* kv_pages, const int* page_tables,
                                      int page_table_stride, int page_size, int n_seqs, const int* cu_seqlens, void* stream);
+/* Prefill attention of NEW rows over the paged cache (chunked prefill, continuing a cached sequence): replaces torch.cat of the
+ * past K/V (modeling_llama.py:451-456) + flash_attn_func(causal=True) with q_len < kv_len, whose causal mask is aligned
+ * bottom-right (:564-566), for the rows prepare_inputs_for_generation keeps after dropping the cached prefix (:1112-1149).
+ * Rows [cu_q[b], cu_q[b+1]) of q (device int32 [n_seqs+1]) are sequence b's new rows at positions start_pos[b] + i (device
+ * int32 [n_seqs]); the row at position p attends to positions 0..p of its sequence, read from ONE layer's kv_pages
+ * ([n_pages, 2, page_size, nkv, hd], as srgpt_rope_kv_append_bf16 describes) through page_tables + b * page_table_stride.
+ * The new rows' own K/V must already be appended (srgpt_rope_kv_append_varlen_bf16).  max_q_len (longest chunk) and
+ * max_ctx_len (largest start_pos[b] + chunk length) are host bounds used for the grid only.  head_dim 128, page_size 16,
+ * n_heads / n_kv_heads <= 8.  q / out: rows [.., q_ld] / [.., o_ld] (e.g. the q columns of the fused qkv buffer).
+ * workspace: fp32 partials of the context split, srgpt_attention_prefill_paged_workspace() bytes (0 = no split for this shape),
+ * 16-byte aligned; NULL runs without a split. */
+long long srgpt_attention_prefill_paged_workspace(int n_seqs, int max_q_len, int max_ctx_len, int n_heads, int n_kv_heads);
+int srgpt_attention_prefill_paged_bf16(const void* q, int q_ld, void* out, int o_ld, const void* kv_pages, const int* page_tables,
+                                       int page_table_stride, int page_size, int n_seqs, const int* cu_q, const int* start_pos,
+                                       int max_q_len, int max_ctx_len, int n_heads, int n_kv_heads, int head_dim, float scale,
+                                       void* workspace, long long workspace_bytes, void* stream);
 /* Decode attention for ONE new token over the paged cache (replaces torch.cat of the cache +
  * flash_attn_func with q_len 1, modeling_llama.py:451-456,564).  q: [nh*hd] bf16 (already rotated),
  * kv_len_minus1: device int = position of the new token (its k/v are already in the cache). */
@@ -290,6 +306,14 @@ int srgpt_llama_prefill_layers_bf16(void* x, const srgpt_llama_layer_weights* la
                                     float eps, const void* cos_tab, const void* sin_tab, const int* start_pos,
                                     const int* page_tables, int page_size, int n_seqs, const int* cu_seqlens, int max_seqlen,
                                     int page_table_stride, void* stream);
+/* The same layers over new rows that CONTINUE sequences already in the cache (chunked prefill, a follow-up turn): S rows of
+ * n_seqs chunks packed back to back (cu_seqlens, max_seqlen as above), chunk b at positions start_pos[b].., attention over all
+ * cached positions through srgpt_attention_prefill_paged_bf16 (max_ctx_len, ws_split / ws_split_bytes = its bound and workspace). */
+int srgpt_llama_prefill_layers_paged_bf16(void* x, const srgpt_llama_layer_weights* layers, int n_layers, void* ws_h, void* ws_qkv,
+                                          void* ws_attn, void* ws_act, void* ws_split, long long ws_split_bytes, int S, int H, int n_heads,
+                                          int n_kv_heads, int head_dim, int I, float eps, const void* cos_tab, const void* sin_tab,
+                                          const int* start_pos, const int* page_tables, int page_table_stride, int page_size, int n_seqs,
+                                          const int* cu_seqlens, int max_seqlen, int max_ctx_len, void* stream);
 /* One whole decode step (5 kernels per layer + lm_head + argmax), h [H] in/out = residual stream of the new token. */
 int srgpt_llama_decode_step_bf16(void* h, const srgpt_llama_layer_weights* layers, int n_layers, void* q_buf, void* attn_buf,
                                  void* act_buf, int H, int n_heads, int n_kv_heads, int head_dim, int I, float eps,

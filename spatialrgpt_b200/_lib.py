@@ -51,6 +51,8 @@ SIGNATURES = {
     "srgpt_attention_prefill_varlen_bf16": (ci, [vp, vp, vp, vp, ci, ci, ci, ci, vp, ci, ci, ci, ci, ci, cf, ci, vp]),
     "srgpt_rope_kv_append_bf16": (ci, [vp, ci, ci, ci, ci, vp, vp, vp, vp, vp, ci, vp]),
     "srgpt_rope_kv_append_varlen_bf16": (ci, [vp, ci, ci, ci, ci, vp, vp, vp, vp, vp, ci, ci, ci, vp, vp]),
+    "srgpt_attention_prefill_paged_workspace": (cll, [ci, ci, ci, ci, ci]),
+    "srgpt_attention_prefill_paged_bf16": (ci, [vp, ci, vp, ci, vp, vp, ci, ci, ci, vp, vp, ci, ci, ci, ci, ci, cf, vp, cll, vp]),
     "srgpt_attention_decode_bf16": (ci, [vp, vp, vp, vp, ci, vp, ci, ci, ci, cf, vp]),
     "srgpt_gemv_bf16": (ci, [vp, vp, ci, vp, ci, ci, vp, cf, vp, ci, ci, ci, ci, vp, vp, vp, vp, vp, ci, vp]),
     "srgpt_lm_head_workspace": (cll, [ci]),
@@ -76,6 +78,8 @@ SIGNATURES = {
     "srgpt_siglip_layers_bf16": (ci, [vp, vp, ci, vp, vp, vp, vp, ci, ci, ci, ci, ci, cf, vp]),
     "srgpt_vit_layers_bf16": (ci, [vp, vp, ci, vp, vp, vp, vp, ci, ci, ci, ci, ci, cf, ci, vp]),
     "srgpt_llama_prefill_layers_bf16": (ci, [vp, vp, ci, vp, vp, vp, vp, ci, ci, ci, ci, ci, ci, cf, vp, vp, vp, vp, ci, ci, vp, ci, ci, vp]),
+    "srgpt_llama_prefill_layers_paged_bf16": (ci, [vp, vp, ci, vp, vp, vp, vp, vp, cll, ci, ci, ci, ci, ci, ci, cf, vp, vp, vp, vp, ci, ci, ci,
+                                                   vp, ci, ci, vp]),
     "srgpt_llama_decode_step_bf16": (ci, [vp, vp, ci, vp, vp, vp, ci, ci, ci, ci, ci, cf, vp, vp, vp, vp, ci, vp, vp, ci, vp, vp, vp, vp,
                                           vp, vp]),
 }

@@ -6,7 +6,11 @@
 //     and <1 % of the Llama prefill FLOPs at S~260, the GEMMs are on tcgen05 already.)
 //   * rope_kv_append_kernel : RoPE on q,k + paged KV-cache append for the prompt tokens.
 //   * attn_decode_kernel    : one-token attention over the paged KV cache.
+//   * attn_prefill_paged_kernel : new prompt rows over the paged KV cache (chunked prefill / continuing a cached
+//     sequence); mma.sync, chosen over tcgen05 for its latency / bytes-bound shapes (see the comment above the kernel).
 // Reference: modeling_llama.py:405-566 (LlamaFlashAttention2), :160-191 (RoPE); HF SiglipAttention.
+#include <algorithm>
+
 #include "common.cuh"
 #include "srgpt_b200.h"
 
@@ -537,6 +541,248 @@ attn_decode_gqa_kernel(const bf16* __restrict__ q, int q_ld, bf16* __restrict__ 
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Prefill attention over the PAGED cache: new prompt rows of a sequence attend to every earlier position, whether it was
+// written by this chunk or by an earlier prefill / decode (chunked prefill, continuing a cached conversation).  The reference
+// concatenates the past K/V (modeling_llama.py:451-456) and calls flash_attn_func(causal=True) with q_len < kv_len, i.e. the
+// causal mask aligned bottom-right (:564-566); prepare_inputs_for_generation drops the cached prefix (:1112-1149).
+//
+// Rows [cu_q[b], cu_q[b+1]) of q are sequence b's new rows at positions start_pos[b] + i; their K/V are already in the pages
+// (srgpt_rope_kv_append_varlen_bf16).  Row at position p attends to positions 0..p, read through page_tables[b].
+//
+// Work split.  One CTA serves all G query heads of a kv head: the 64 rows of the MMA tile are G x (64 / G) (query row, head)
+// pairs, packed row pr = (row q0 + pr / G, head kvh * G + pr % G), so every K/V tile is read once per group and q tile (GQA
+// shares the pass like attn_decode_gqa_kernel).  When seqs x kv heads x q tiles is far below one wave (a 40-row follow-up turn
+// of Llama-3-8B is 24 CTAs) the context is split over CTAs; each split writes fp32 (O, m, l) and attn_paged_combine_kernel
+// merges them in split order (deterministic, no atomics, graph-safe).
+// mma.sync m16n8k16 + cp.async page loads, same rounding as attn_prefill_kernel (fp32 scores and online softmax, P rounded to
+// the element type before P.V, the output rounded once).  tcgen05 is not used: the follow-up shape is ~0.3 GFLOP and 2 MB of
+// K/V per layer (latency / bytes bound, and page-granular gathers do not map onto one TMA box), and a 512-row chunk at the end of
+// a 4k context (~32 GFLOP per layer) is a rare shape next to the GEMMs of the same chunk.
+// ---------------------------------------------------------------------------------------------
+constexpr int PG_PAGE = 16;
+constexpr int PG_SPLIT_BELOW = 74;   // split the context when the grid has at most half a wave of CTAs...
+constexpr int PG_SPLIT_TARGET = 148; // ...up to about one wave (the B200's SM count; fixed so the workspace size is host arithmetic)
+
+using PagedSmem = Smem<128, 128>;
+
+// K (which = 0) or V (which = 1) rows of positions [kv0, kv0 + 64) of kv head kvh; positions >= kv_len are zero-filled (no
+// page-table read past the sequence's reserved pages)
+__device__ __forceinline__ void load_kv_paged(bf16 (*dst)[PagedSmem::LD], const bf16* __restrict__ kv_pages, const int* __restrict__ pt,
+                                              size_t row_stride, int kvh, int which, int kv0, int kv_len) {
+  for (int i = threadIdx.x; i < BN * 16; i += NTHREADS) {
+    const int r = i >> 4, c = i & 15;
+    const int j = kv0 + r;
+    if (j < kv_len) {
+      const int page = __ldg(pt + j / PG_PAGE);
+      cp_async16(&dst[r][c * 8], kv_pages + (((size_t)page * 2 + which) * PG_PAGE + (j % PG_PAGE)) * row_stride + kvh * 128 + c * 8);
+    } else {
+      *reinterpret_cast<uint4*>(&dst[r][c * 8]) = make_uint4(0, 0, 0, 0);
+    }
+  }
+}
+
+__global__ void __launch_bounds__(NTHREADS)
+attn_prefill_paged_kernel(const bf16* __restrict__ q, int q_ld, bf16* __restrict__ out, int o_ld, const bf16* __restrict__ kv_pages,
+                          const int* __restrict__ page_tables, int pt_stride, const int* __restrict__ cu_q, const int* __restrict__ start_pos,
+                          int n_heads, int n_kv_heads, int group, int n_split, int tiles_per_split, float* __restrict__ ws_o,
+                          float* __restrict__ ws_ml, int ws_rows, float scale_log2) {
+  constexpr int HD = 128;
+  using S = PagedSmem;
+  extern __shared__ __align__(16) uint8_t smem_raw[];
+  S& sm = *reinterpret_cast<S*>(smem_raw);
+
+  const int qt = blockIdx.x, kvh = blockIdx.y, b = blockIdx.z / n_split, split = blockIdx.z % n_split;
+  const int QR = BM / group;  // query rows per tile
+  const int row_base = cu_q[b], q_len = cu_q[b + 1] - row_base;
+  const int q0 = qt * QR;
+  if (q0 >= q_len) return;  // grid.x covers the longest chunk
+  const int sp = start_pos[b];
+  const int kv_len = sp + min(q0 + QR, q_len);  // positions [0, kv_len) are visible to some row of this tile
+  const int ntiles = (kv_len + BN - 1) / BN;
+  const int t_begin = min(split * tiles_per_split, ntiles);
+  const int t_end = split == n_split - 1 ? ntiles : min(ntiles, t_begin + tiles_per_split);
+  const int* pt = page_tables + (size_t)b * pt_stride;
+  const size_t row_stride = (size_t)n_kv_heads * HD;
+
+  for (int i = threadIdx.x; i < BM * 16; i += NTHREADS) {
+    const int pr = i >> 4, c = i & 15, qi = pr / group;
+    if (pr < QR * group && q0 + qi < q_len)
+      cp_async16(&sm.q[pr][c * 8], q + (size_t)(row_base + q0 + qi) * q_ld + (kvh * group + pr % group) * HD + c * 8);
+    else
+      *reinterpret_cast<uint4*>(&sm.q[pr][c * 8]) = make_uint4(0, 0, 0, 0);
+  }
+  if (t_begin < t_end) {
+    load_kv_paged(sm.k[0], kv_pages, pt, row_stride, kvh, 0, t_begin * BN, kv_len);
+    load_kv_paged(sm.v[0], kv_pages, pt, row_stride, kvh, 1, t_begin * BN, kv_len);
+  }
+  cp_async_commit();
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int lr = lane & 7, lmat = lane >> 3;
+  const int g = lane >> 2, t4 = lane & 3;
+  // this thread's two packed rows (pr, pr + 8): query position, or -1 for a padding row (everything masked)
+  int prow[2], ppos[2];
+#pragma unroll
+  for (int r = 0; r < 2; ++r) {
+    const int pr = warp * 16 + g + r * 8, qi = pr / group;
+    const bool ok = pr < QR * group && q0 + qi < q_len;
+    prow[r] = pr;
+    ppos[r] = ok ? sp + q0 + qi : -1;
+  }
+
+  float o[HD / 8][4];
+#pragma unroll
+  for (int i = 0; i < HD / 8; ++i) o[i][0] = o[i][1] = o[i][2] = o[i][3] = 0.f;
+  float m_run[2] = {-INFINITY, -INFINITY}, l_run[2] = {0.f, 0.f};
+  uint32_t qf[HD / 16][4];
+
+  if (t_begin == t_end) cp_async_wait<0>();
+  for (int j = t_begin; j < t_end; ++j) {
+    const int cur = (j - t_begin) & 1;
+    if (j + 1 < t_end) {
+      load_kv_paged(sm.k[cur ^ 1], kv_pages, pt, row_stride, kvh, 0, (j + 1) * BN, kv_len);
+      load_kv_paged(sm.v[cur ^ 1], kv_pages, pt, row_stride, kvh, 1, (j + 1) * BN, kv_len);
+      cp_async_commit();
+      cp_async_wait<1>();
+    } else {
+      cp_async_wait<0>();
+    }
+    __syncthreads();
+    if (j == t_begin) {
+#pragma unroll
+      for (int kk = 0; kk < HD / 16; ++kk)
+        ldmatrix_x4(qf[kk], &sm.q[warp * 16 + lr + (lmat & 1) * 8][kk * 16 + (lmat >> 1) * 8]);
+    }
+    // ---- S = Q K^T (16 packed rows x 64 positions per warp)
+    float s[BN / 8][4];
+#pragma unroll
+    for (int i = 0; i < BN / 8; ++i) s[i][0] = s[i][1] = s[i][2] = s[i][3] = 0.f;
+#pragma unroll
+    for (int np = 0; np < BN / 16; ++np) {
+#pragma unroll
+      for (int kk = 0; kk < HD / 16; ++kk) {
+        uint32_t bfr[4];
+        ldmatrix_x4(bfr, &sm.k[cur][np * 16 + lr + (lmat >> 1) * 8][kk * 16 + (lmat & 1) * 8]);
+        mma_bf16_16816(s[2 * np], qf[kk], bfr[0], bfr[1]);
+        mma_bf16_16816(s[2 * np + 1], qf[kk], bfr[2], bfr[3]);
+      }
+    }
+    // ---- scale, causal mask (bottom-right aligned: position p sees 0..p), online softmax
+    float mx[2] = {-INFINITY, -INFINITY};
+#pragma unroll
+    for (int nb = 0; nb < BN / 8; ++nb) {
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const int kv = j * BN + nb * 8 + 2 * t4 + (e & 1);
+        float val = s[nb][e] * scale_log2;
+        if (kv > ppos[e >> 1]) val = -INFINITY;
+        s[nb][e] = val;
+        mx[e >> 1] = fmaxf(mx[e >> 1], val);
+      }
+    }
+    float alpha[2], m_new[2];
+#pragma unroll
+    for (int r = 0; r < 2; ++r) {
+      mx[r] = fmaxf(mx[r], __shfl_xor_sync(0xffffffffu, mx[r], 1));
+      mx[r] = fmaxf(mx[r], __shfl_xor_sync(0xffffffffu, mx[r], 2));
+      m_new[r] = fmaxf(m_run[r], mx[r]);
+      const float m_use = (m_new[r] == -INFINITY) ? 0.f : m_new[r];
+      alpha[r] = exp2f(m_run[r] - m_use);
+      m_run[r] = m_new[r];
+      m_new[r] = m_use;
+    }
+    float rs[2] = {0.f, 0.f};
+#pragma unroll
+    for (int nb = 0; nb < BN / 8; ++nb) {
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const float p = exp2f(s[nb][e] - m_new[e >> 1]);
+        s[nb][e] = p;
+        rs[e >> 1] += p;
+      }
+    }
+#pragma unroll
+    for (int r = 0; r < 2; ++r) l_run[r] = l_run[r] * alpha[r] + rs[r];
+#pragma unroll
+    for (int i = 0; i < HD / 8; ++i) {
+      o[i][0] *= alpha[0]; o[i][1] *= alpha[0];
+      o[i][2] *= alpha[1]; o[i][3] *= alpha[1];
+    }
+    // ---- O += P V
+#pragma unroll
+    for (int kk = 0; kk < BN / 16; ++kk) {
+      uint32_t a[4];
+      a[0] = pack_bf16x2(s[2 * kk][0], s[2 * kk][1]);
+      a[1] = pack_bf16x2(s[2 * kk][2], s[2 * kk][3]);
+      a[2] = pack_bf16x2(s[2 * kk + 1][0], s[2 * kk + 1][1]);
+      a[3] = pack_bf16x2(s[2 * kk + 1][2], s[2 * kk + 1][3]);
+#pragma unroll
+      for (int dp = 0; dp < HD / 16; ++dp) {
+        uint32_t bfr[4];
+        ldmatrix_x4_trans(bfr, &sm.v[cur][kk * 16 + lr + (lmat & 1) * 8][dp * 16 + (lmat >> 1) * 8]);
+        mma_bf16_16816(o[2 * dp], a, bfr[0], bfr[1]);
+        mma_bf16_16816(o[2 * dp + 1], a, bfr[2], bfr[3]);
+      }
+    }
+    __syncthreads();  // all warps done with buffer `cur` before it is refilled
+  }
+
+#pragma unroll
+  for (int r = 0; r < 2; ++r) {
+    l_run[r] += __shfl_xor_sync(0xffffffffu, l_run[r], 1);
+    l_run[r] += __shfl_xor_sync(0xffffffffu, l_run[r], 2);
+  }
+#pragma unroll
+  for (int r = 0; r < 2; ++r) {
+    if (ppos[r] < 0) continue;
+    const int row = row_base + q0 + prow[r] / group, head = kvh * group + prow[r] % group;
+    if (n_split == 1) {
+      const float inv = l_run[r] > 0.f ? 1.f / l_run[r] : 0.f;
+      bf16* ob = out + (size_t)row * o_ld + head * HD;
+#pragma unroll
+      for (int db = 0; db < HD / 8; ++db)
+        *reinterpret_cast<uint32_t*>(ob + db * 8 + 2 * t4) = pack_bf16x2(o[db][2 * r] * inv, o[db][2 * r + 1] * inv);
+    } else if (row < ws_rows) {
+      const size_t slot = ((size_t)split * ws_rows + row) * n_heads + head;
+      float* wo = ws_o + slot * HD;
+#pragma unroll
+      for (int db = 0; db < HD / 8; ++db) *reinterpret_cast<float2*>(wo + db * 8 + 2 * t4) = make_float2(o[db][2 * r], o[db][2 * r + 1]);
+      if (t4 == 0) *reinterpret_cast<float2*>(ws_ml + slot * 2) = make_float2(m_run[r], l_run[r]);
+    }
+  }
+}
+
+// merges the n_split partial results of a row and head in split order: O = sum_s o_s 2^(m_s - M) / sum_s l_s 2^(m_s - M)
+__global__ void __launch_bounds__(128)
+attn_paged_combine_kernel(const float* __restrict__ ws_o, const float* __restrict__ ws_ml, bf16* __restrict__ out, int o_ld,
+                          const int* __restrict__ cu_q, int n_seqs, int n_split, int ws_rows, int n_heads) {
+  const int row = blockIdx.x, head = blockIdx.y, d = threadIdx.x;
+  if (row >= cu_q[n_seqs]) return;
+  float mt = -INFINITY;
+  for (int s = 0; s < n_split; ++s) mt = fmaxf(mt, ws_ml[(((size_t)s * ws_rows + row) * n_heads + head) * 2]);
+  float lt = 0.f, at = 0.f;
+  for (int s = 0; s < n_split; ++s) {
+    const size_t slot = ((size_t)s * ws_rows + row) * n_heads + head;
+    const float m = ws_ml[slot * 2];
+    const float w = m == -INFINITY ? 0.f : exp2f(m - mt);
+    lt += ws_ml[slot * 2 + 1] * w;
+    at += ws_o[slot * 128 + d] * w;
+  }
+  out[(size_t)row * o_ld + head * 128 + d] = f2e(lt > 0.f ? at / lt : 0.f);
+}
+
+// context split of the paged kernel; pure host arithmetic (the workspace size must not need a device)
+static int paged_split(int n_seqs, int max_q_len, int max_ctx_len, int n_heads, int n_kv_heads, int* tiles_per_split) {
+  const int group = n_heads / n_kv_heads;
+  const int ctas = n_seqs * n_kv_heads * ceil_div(max_q_len, BM / group);
+  const int kv_tiles = ceil_div(max_ctx_len, BN);
+  int n_split = 1;
+  if (ctas <= PG_SPLIT_BELOW) n_split = std::max(1, std::min(kv_tiles, ceil_div(PG_SPLIT_TARGET, ctas)));
+  *tiles_per_split = ceil_div(kv_tiles, n_split);
+  return ceil_div(kv_tiles, *tiles_per_split);  // no empty trailing split
+}
+
 template <int HD, int HDP, bool CAUSAL>
 static int launch_prefill(const void* q, const void* k, const void* v, void* out, int q_ld, int kv_ld, int o_ld, int batch,
                           int seqlen, const int* cu_seqlens, int n_heads, int n_kv_heads, float scale, cudaStream_t st) {
@@ -660,6 +906,65 @@ extern "C" __attribute__((visibility("default"))) int srgpt_attention_decode_bf1
   SRGPT_CHECK_CUDA(cudaLaunchKernelEx(&cfg, attn::attn_decode_kernel, reinterpret_cast<const bf16*>(q), reinterpret_cast<bf16*>(out),
                                       reinterpret_cast<const bf16*>(kv_pages), page_table, page_size, kv_len_minus1, n_kv_heads,
                                       n_heads / n_kv_heads, scale * 1.4426950408889634f, trace_next_slot(), no_prefetch ? 0 : 1, 0, 0, 0, 0));
+  return SRGPT_OK;
+}
+
+static bool paged_args_ok(int n_seqs, int max_q_len, int max_ctx_len, int n_heads, int n_kv_heads) {
+  return n_seqs > 0 && n_seqs <= 65535 / attn::PG_SPLIT_TARGET && max_q_len > 0 && max_ctx_len >= max_q_len && n_heads > 0 && n_kv_heads > 0 &&
+         (n_heads % n_kv_heads) == 0 && n_heads / n_kv_heads <= 8;
+}
+
+extern "C" __attribute__((visibility("default"))) long long srgpt_attention_prefill_paged_workspace(int n_seqs, int max_q_len, int max_ctx_len,
+                                                                                                    int n_heads, int n_kv_heads) {
+  if (!paged_args_ok(n_seqs, max_q_len, max_ctx_len, n_heads, n_kv_heads)) return -1;
+  int tps = 0;
+  const int n_split = attn::paged_split(n_seqs, max_q_len, max_ctx_len, n_heads, n_kv_heads, &tps);
+  if (n_split == 1) return 0;
+  return (long long)n_split * n_seqs * max_q_len * n_heads * (128 + 2) * (long long)sizeof(float);
+}
+
+extern "C" __attribute__((visibility("default"))) int srgpt_attention_prefill_paged_bf16(const void* q, int q_ld, void* out, int o_ld, const void* kv_pages,
+                                                                                         const int* page_tables, int page_table_stride, int page_size, int n_seqs,
+                                                                                         const int* cu_q, const int* start_pos, int max_q_len, int max_ctx_len,
+                                                                                         int n_heads, int n_kv_heads, int head_dim, float scale, void* workspace,
+                                                                                         long long workspace_bytes, void* stream) {
+  SRGPT_CHECK_ARG(q && out && kv_pages && page_tables && cu_q && start_pos);
+  SRGPT_CHECK_ARG(paged_args_ok(n_seqs, max_q_len, max_ctx_len, n_heads, n_kv_heads) && page_table_stride > 0);
+  SRGPT_CHECK_ARG(aligned16(q) && aligned16(kv_pages) && (q_ld % 8) == 0 && q_ld >= n_heads * head_dim && o_ld >= n_heads * head_dim);
+  SRGPT_CHECK_ARG((o_ld % 2) == 0 && (reinterpret_cast<uintptr_t>(out) & 3) == 0);
+  if (head_dim != 128 || page_size != attn::PG_PAGE) {
+    set_last_error("srgpt_attention_prefill_paged_bf16: head_dim %d / page_size %d unsupported (128 / 16 only)", head_dim, page_size);
+    return SRGPT_ERR_UNSUPPORTED;
+  }
+  int tps = 0;
+  int n_split = attn::paged_split(n_seqs, max_q_len, max_ctx_len, n_heads, n_kv_heads, &tps);
+  const long long need = srgpt_attention_prefill_paged_workspace(n_seqs, max_q_len, max_ctx_len, n_heads, n_kv_heads);
+  if (workspace == nullptr) {  // no workspace: one CTA walks the whole context
+    n_split = 1;
+    tps = ceil_div(max_ctx_len, attn::BN);
+  } else {
+    SRGPT_CHECK_ARG(workspace_bytes >= need && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0);
+  }
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  static bool configured = false;
+  if (!configured) {
+    SRGPT_CHECK_CUDA(cudaFuncSetAttribute(attn::attn_prefill_paged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(attn::PagedSmem)));
+    configured = true;
+  }
+  const int group = n_heads / n_kv_heads;
+  const int ws_rows = n_seqs * max_q_len;
+  float* ws_o = reinterpret_cast<float*>(workspace);
+  float* ws_ml = ws_o == nullptr ? nullptr : ws_o + (size_t)n_split * ws_rows * n_heads * 128;
+  const dim3 grid(ceil_div(max_q_len, attn::BM / group), n_kv_heads, n_seqs * n_split);
+  attn::attn_prefill_paged_kernel<<<grid, attn::NTHREADS, sizeof(attn::PagedSmem), st>>>(
+      reinterpret_cast<const bf16*>(q), q_ld, reinterpret_cast<bf16*>(out), o_ld, reinterpret_cast<const bf16*>(kv_pages), page_tables,
+      page_table_stride, cu_q, start_pos, n_heads, n_kv_heads, group, n_split, tps, ws_o, ws_ml, ws_rows, scale * 1.4426950408889634f);
+  SRGPT_CHECK_LAUNCH();
+  if (n_split > 1) {
+    attn::attn_paged_combine_kernel<<<dim3(ws_rows, n_heads), 128, 0, st>>>(ws_o, ws_ml, reinterpret_cast<bf16*>(out), o_ld, cu_q, n_seqs, n_split,
+                                                                          ws_rows, n_heads);
+    SRGPT_CHECK_LAUNCH();
+  }
   return SRGPT_OK;
 }
 

@@ -76,6 +76,36 @@ extern "C" __attribute__((visibility("default"))) int srgpt_llama_prefill_layers
   return SRGPT_OK;
 }
 
+// The same layer sequence for new rows that continue sequences already in the cache (chunked prefill, a follow-up turn): RoPE
+// and the KV append at start_pos[b] + i, then attention of the new rows over ALL cached positions of their sequence through
+// the page tables (srgpt_attention_prefill_paged_bf16; modeling_llama.py:451-456 + 564-566 with q_len < kv_len).
+extern "C" __attribute__((visibility("default"))) int srgpt_llama_prefill_layers_paged_bf16(
+    void* x, const srgpt_llama_layer_weights* layers, int n_layers, void* ws_h, void* ws_qkv, void* ws_attn, void* ws_act, void* ws_split,
+    long long ws_split_bytes, int S, int H, int n_heads, int n_kv_heads, int head_dim, int I, float eps, const void* cos_tab, const void* sin_tab,
+    const int* start_pos, const int* page_tables, int page_table_stride, int page_size, int n_seqs, const int* cu_seqlens, int max_seqlen,
+    int max_ctx_len, void* stream) {
+  SRGPT_CHECK_ARG(x && layers && ws_h && ws_qkv && ws_attn && ws_act && start_pos && page_tables && cu_seqlens);
+  SRGPT_CHECK_ARG(n_layers >= 0 && S > 0 && H > 0 && n_heads > 0 && n_kv_heads > 0 && head_dim > 0 && I > 0);
+  SRGPT_CHECK_ARG(n_seqs >= 1 && max_seqlen >= 1 && max_seqlen <= S && max_ctx_len >= max_seqlen && page_table_stride > 0);
+  const int qd = n_heads * head_dim, kd = n_kv_heads * head_dim, nqkv = qd + 2 * kd;
+  const float scale = 1.0f / sqrtf((float)head_dim);
+  for (int l = 0; l < n_layers; ++l) {
+    const srgpt_llama_layer_weights& w = layers[l];
+    SRGPT_TRY(srgpt_rmsnorm_bf16(x, H, w.in_norm, ws_h, H, S, H, eps, stream));
+    SRGPT_TRY(srgpt_gemm_bf16(ws_h, H, w.qkv_w, H, ws_qkv, nqkv, S, nqkv, H, nullptr, nullptr, 0, 0, SRGPT_EPI_NONE, 0, stream));
+    SRGPT_TRY(srgpt_rope_kv_append_varlen_bf16(ws_qkv, S, n_heads, n_kv_heads, head_dim, cos_tab, sin_tab, start_pos, w.kv_pages, page_tables,
+                                               page_table_stride, page_size, n_seqs, cu_seqlens, stream));
+    SRGPT_TRY(srgpt_attention_prefill_paged_bf16(ws_qkv, nqkv, ws_attn, qd, w.kv_pages, page_tables, page_table_stride, page_size, n_seqs, cu_seqlens,
+                                                 start_pos, max_seqlen, max_ctx_len, n_heads, n_kv_heads, head_dim, scale, ws_split, ws_split_bytes,
+                                                 stream));
+    SRGPT_TRY(srgpt_gemm_bf16(ws_attn, qd, w.o_w, qd, x, H, S, H, qd, nullptr, x, H, 0, SRGPT_EPI_BIAS_RESIDUAL, 0, stream));
+    SRGPT_TRY(srgpt_rmsnorm_bf16(x, H, w.post_norm, ws_h, H, S, H, eps, stream));
+    SRGPT_TRY(srgpt_gemm_bf16(ws_h, H, w.gateup_w, H, ws_act, I, S, 2 * I, H, nullptr, nullptr, 0, 0, SRGPT_EPI_SWIGLU, 0, stream));
+    SRGPT_TRY(srgpt_gemm_bf16(ws_act, I, w.down_w, I, x, H, S, H, I, nullptr, x, H, 0, SRGPT_EPI_BIAS_RESIDUAL, 0, stream));
+  }
+  return SRGPT_OK;
+}
+
 extern "C" __attribute__((visibility("default"))) int srgpt_llama_decode_step_bf16(void* h, const srgpt_llama_layer_weights* layers, int n_layers, void* q_buf, void* attn_buf,
                                                                                      void* act_buf, int H, int n_heads, int n_kv_heads, int head_dim, int I, float eps,
                                                                                      const void* cos_tab, const void* sin_tab, int* pos, const int* page_table,

@@ -122,6 +122,14 @@ class LlamaDecoder:
         self.sample_logits: Optional[torch.Tensor] = None
         self.sample_seed = 0
         self.sample_seed_dev = torch.zeros(1, dtype=torch.int64, device=dev)  # device copy: the captured graph reads the seed at run time
+        # bumped by every call that releases or re-lays out the cached pages: a KV handle filled in an older epoch is stale
+        self.kv_epoch = 0
+
+    def release_all(self) -> None:
+        """Drop every cached sequence (the start of an unrelated request)."""
+        for b in range(len(self.cache.owned)):
+            self.cache.release(b)
+        self.kv_epoch += 1
 
     # ---------------------------------------------------------------------------------------------
     @ops.in_own_dtype
@@ -140,6 +148,7 @@ class LlamaDecoder:
             raise RuntimeError(f"KV cache for {n_seqs} x {tokens_per_seq} tokens needs {need_pages * per_page >> 20} MiB, not available")
         self._graph = None
         self._graph_sample = None
+        self.kv_epoch += 1
         n_pages_old, n_seqs_old = c.n_pages, len(c.owned)
         self.cache = None
         del c
@@ -158,8 +167,10 @@ class LlamaDecoder:
 
     @ops.in_own_dtype
     def prefill_hidden(self, inputs_embeds: torch.Tensor, seq: int = 0, start_pos: int = 0) -> torch.Tensor:
-        """Run all layers over one sequence's prompt rows [S, H]; fills the KV cache; returns the
-        final-layer residual stream [S, H] (before the final norm)."""
+        """Run all layers over one sequence's prompt rows [S, H] at positions [start_pos, start_pos + S); fills the KV cache;
+        returns the final-layer residual stream [S, H] (before the final norm).  With start_pos > 0 the rows attend to the
+        positions [0, start_pos) this sequence already holds in the cache (srgpt_llama_prefill_layers_paged_bf16), so calling it
+        chunk by chunk is chunked prefill; start_pos == 0 is the one-shot prompt path."""
         d, w = self.dims, self.w
         S = inputs_embeds.shape[0]
         if start_pos + S > self.max_seq_len:
@@ -168,9 +179,11 @@ class LlamaDecoder:
         sp = torch.tensor([start_pos], dtype=torch.int32, device=self.device)
         pt = self.cache.page_tables[seq]
         x = inputs_embeds.to(self.dtype).contiguous().clone()
-        if start_pos != 0:
-            raise NotImplementedError("chunked prefill (prompt attention over cached pages) is a next-round item")
-        return ops.llama_prefill_layers(x, self._layer_array, d.num_hidden_layers, d, self.cos, self.sin, sp, pt, PAGE_SIZE)
+        if start_pos == 0:
+            return ops.llama_prefill_layers(x, self._layer_array, d.num_hidden_layers, d, self.cos, self.sin, sp, pt, PAGE_SIZE)
+        cu = torch.tensor([0, S], dtype=torch.int32, device=self.device)
+        return ops.llama_prefill_layers_paged(x, self._layer_array, d.num_hidden_layers, d, self.cos, self.sin, sp, self.cache.page_tables[seq:seq + 1],
+                                              PAGE_SIZE, cu, S, start_pos + S)
 
     @ops.in_own_dtype
     def prefill_packed(self, packed_embeds: torch.Tensor, seq_lens: List[int]) -> torch.Tensor:
@@ -271,10 +284,15 @@ class LlamaDecoder:
     @torch.no_grad()
     @ops.in_own_dtype
     def generate_from_embeds(self, inputs_embeds: torch.Tensor, max_new_tokens: int, eos_token_ids=None, stopping_fn=None,
-                             use_graph: bool = True, return_logits: bool = False, seq: int = 0, sampling=None):
+                             use_graph: bool = True, return_logits: bool = False, seq: int = 0, sampling=None, prefix_len: int = 0):
         """Greedy (or, with ``sampling=dict(temperature, top_p, seed)``, nucleus-sampled) decoding started from prompt
         embeddings [S, H].  Returns LongTensor [n_new] (and fp32 logits [n_new, V] when return_logits).
-        ``stopping_fn(ids_so_far: LongTensor) -> bool``."""
+        ``stopping_fn(ids_so_far: LongTensor) -> bool``.
+
+        ``prefix_len`` = L > 0 continues what sequence `seq` already caches: its pages for positions [0, L) are kept (the caller
+        has checked that they hold exactly inputs_embeds[:L]) and only rows [L, S) are prefilled, at position L.  L = 0 releases
+        every cached sequence first.  After S prompt rows and n returned tokens the cache holds the final KV of positions
+        [0, S + n - 1): see cached_length()."""
         d, w = self.dims, self.w
         S = inputs_embeds.shape[0]
         if max_new_tokens < 1:
@@ -286,21 +304,36 @@ class LlamaDecoder:
         eos = set()
         if eos_token_ids is not None:
             eos = set(int(e) for e in (eos_token_ids if isinstance(eos_token_ids, (list, tuple, set)) else [eos_token_ids]))
-        for b in range(len(self.cache.owned)):  # a previous batched generate leaves pages owned by sequences 1..B-1
-            self.cache.release(b)
+        if not 0 <= prefix_len < S:
+            raise ValueError(f"prefix_len {prefix_len} must lie in [0, {S}): at least one prompt row is prefilled")
+        if prefix_len == 0:
+            self.release_all()  # a previous batched generate leaves pages owned by sequences 1..B-1
+        else:
+            for b in range(len(self.cache.owned)):
+                if b != seq:
+                    self.cache.release(b)
         self.cache.reserve(seq, S + max_new_tokens)
-        hidden = self.prefill_hidden(inputs_embeds, seq, 0)
+        hidden = self.prefill_hidden(inputs_embeds[prefix_len:], seq, prefix_len)
         logits = torch.empty((max_new_tokens, d.vocab_size), dtype=torch.float32, device=self.device) if return_logits else None
         # first token: final norm + lm_head + argmax on the last prompt row; afterwards pos == S
         self.pos.fill_(S - 1)
         self.step.zero_()
         sample = self._set_sampling(sampling)
         first_logits = logits[0] if logits is not None else (self._sample_buffer() if sample else None)
-        ops.lm_head_argmax(hidden[S - 1], w.lm_head, w.norm, d.rms_norm_eps, self.lm_ws, self.out_ids, self.step, self.pos,
+        ops.lm_head_argmax(hidden[S - 1 - prefix_len], w.lm_head, w.norm, d.rms_norm_eps, self.lm_ws, self.out_ids, self.step, self.pos,
                            embed_table=w.embed, next_x=self.h, logits_out=first_logits)
         if sample:
             ops.sample_top_p(first_logits, self.sample_params, self.sample_seed_dev, self.step, -1, self.out_ids, w.embed, self.h)
         return self._decode_loop(seq, 1, max_new_tokens, eos, stopping_fn, use_graph, logits, sample)
+
+    @staticmethod
+    def cached_length(prompt_len: int, n_new: int) -> int:
+        """Positions whose KV is final after generate_from_embeds returned n_new >= 1 tokens for a prompt of prompt_len rows.
+        Decode step k (k = 1..n_new-1, _decode_loop) feeds token k-1 at position prompt_len + k - 1, so positions
+        [0, prompt_len + n_new - 1) are written by the prompt and the kept steps; the last returned token was never fed.  On an
+        EOS / stopping-criteria stop the loop may have run ONE speculative step past the stop, which wrote slot
+        prompt_len + n_new - 1 only; that slot is outside the cached length, and the next prefill overwrites it."""
+        return prompt_len + n_new - 1 if n_new > 0 else prompt_len
 
     def _decode_loop(self, seq: int, n: int, max_new_tokens: int, eos, stopping_fn, use_graph: bool, logits, sample: bool = False):
         """Steps n..max_new_tokens-1 of sequence `seq` (greedy, or sampled); pos / step / h / out_ids[:n] are already set."""
@@ -501,8 +534,7 @@ class LlamaDecoder:
         if eos_token_ids is not None:
             eos = [int(e) for e in (eos_token_ids if isinstance(eos_token_ids, (list, tuple, set)) else [eos_token_ids])]
         n_cand = max(2, 1 + len(eos)) * k
-        for b in range(len(self.cache.owned)):
-            self.cache.release(b)
+        self.release_all()
         self.ensure_capacity(k, S + max_new_tokens)
         self.cache.reserve_many([S + max_new_tokens] * k)
         hidden = self.prefill_packed(inputs_embeds.to(self.dtype).repeat(k, 1), [S] * k)
@@ -617,8 +649,7 @@ class LlamaDecoder:
         eos = set()
         if eos_token_ids is not None:
             eos = set(int(e) for e in (eos_token_ids if isinstance(eos_token_ids, (list, tuple, set)) else [eos_token_ids]))
-        for b in range(len(self.cache.owned)):
-            self.cache.release(b)
+        self.release_all()
         self.ensure_capacity(B, max(seq_lens) + max_new_tokens)
         self.cache.reserve_many([n + max_new_tokens for n in seq_lens])
         hidden = self.prefill_packed(packed_embeds, seq_lens)

@@ -2,7 +2,8 @@
 + llava/model/llava_arch.py:252-650) re-built over the sm_100a kernels, keeping its public surface:
 ``generate(input_ids, images=, depths=, masks=, attention_mask=, **generation_kwargs)``, ``forward``,
 ``prepare_inputs_labels_for_multimodal``, ``encode_images``, the ``get_*`` accessors, ``config``,
-``tokenizer``, ``device`` / ``dtype``.  ``LlavaLlamaForCausalLM`` is an alias (the name the north
+``tokenizer``, ``device`` / ``dtype``.  ``past_key_values=`` takes a ``PagedKVCacheHandle`` (kv_handle.py): the KV of a
+previous call stays in the paged cache and only the new rows are prefilled.  ``LlavaLlamaForCausalLM`` is an alias (the name the north
 star and llava/model/builder.py:138 use; the reference never defines it)."""
 from __future__ import annotations
 
@@ -14,6 +15,7 @@ import torch
 from . import ops
 from .config import LlavaConfig
 from .constants import IGNORE_INDEX, IMAGE_TOKEN_INDEX
+from .kv_handle import PagedKVCacheHandle, reusable_prefix
 from .llama_decoder import LlamaDecoder
 from .multimodal_encoder import VisionTower
 from .multimodal_projector import MultimodalProjector
@@ -271,13 +273,53 @@ class LlavaLlamaModel:
         self._last_seq_lens = [x.shape[0] for x in new_embeds]
         return None, ret_pos, ret_am, past_key_values, out, ret_labels
 
+    # ---- KV handles (past_key_values) ------------------------------------------------------------------
+    def _check_handle(self, handle, batch: int, num_beams: int = 1) -> None:
+        if not isinstance(handle, PagedKVCacheHandle):
+            raise NotImplementedError("past_key_values must be a PagedKVCacheHandle; HF tensor caches (DynamicCache / legacy tuples) are "
+                                      "not imported, the KV cache is paged and internal")
+        if batch != 1:
+            raise NotImplementedError("past_key_values is supported for batch 1 only")
+        if num_beams != 1:
+            raise NotImplementedError("past_key_values is not supported with beam search (num_beams > 1)")
+        if type(self.llm).__name__ == "TPLlamaDecoder":
+            raise NotImplementedError("past_key_values is not supported on the tensor-parallel decoder")
+
+    def _forward_continue(self, input_ids, inputs_embeds, attention_mask, handle: PagedKVCacheHandle) -> CausalLMOutputWithPast:
+        """Incremental forward (modeling_llama.py:451-456 + 564-566): the new rows are appended at handle.length and attend to
+        everything the handle's sequence caches; fp32 logits of the new rows only."""
+        llm = self.llm
+        if not handle.is_live_for(llm):
+            raise ValueError("stale past_key_values: the decoder's KV cache has served another request since this handle was filled")
+        if inputs_embeds is None:
+            inputs_embeds = llm.embed_tokens(input_ids).view(*input_ids.shape, -1)
+        if attention_mask is not None and not bool(attention_mask.bool().all()):
+            raise NotImplementedError("padding with past_key_values is not supported")
+        rows = inputs_embeds[0].to(self.dtype)
+        L = handle.length
+        hid = llm.prefill_hidden(rows, 0, L)
+        logits = llm.logits_all(hid)[None]
+        handle.update(llm, torch.cat([handle.rows[:L], rows], 0), L + rows.shape[0])
+        handle.last_reused = L
+        return CausalLMOutputWithPast(logits=logits, past_key_values=handle)
+
     # ---- forward: logits for every position (llava_llama.py:100-192) ----------------------------------
     @torch.no_grad()
     @ops.in_own_dtype
     def forward(self, input_ids=None, images=None, masks=None, depths=None, attention_mask=None, position_ids=None,
                 past_key_values=None, seqlens_in_batch=None, inputs_embeds=None, labels=None, use_cache=None, **kwargs):
+        """``past_key_values=h`` (a PagedKVCacheHandle, batch 1, text rows only): ``input_ids`` are the rows AFTER the cached
+        ones (as prepare_inputs_for_generation feeds them, modeling_llama.py:1112-1149); they are prefilled at h.length over the
+        cached positions, the logits cover the new rows, and h is advanced in place.  An empty handle, or ``use_cache=True``
+        without one (batch 1), runs the full forward and returns the filled handle in ``past_key_values``."""
         if past_key_values is not None:
-            raise NotImplementedError("external past_key_values are not supported; the KV cache is paged and internal")
+            n_batch = (input_ids if inputs_embeds is None else inputs_embeds).shape[0]
+            self._check_handle(past_key_values, n_batch)
+            if past_key_values.length > 0:
+                if images is not None:
+                    raise NotImplementedError("images together with a non-empty past_key_values: the reference re-splices the image into "
+                                              "the new chunk there; pass the whole conversation to generate(..., past_key_values=) instead")
+                return self._forward_continue(input_ids, inputs_embeds, attention_mask, past_key_values)
         if inputs_embeds is None:
             if images is None:
                 inputs_embeds = self.llm.embed_tokens(input_ids).view(*input_ids.shape, -1)
@@ -297,8 +339,7 @@ class LlavaLlamaModel:
                     raise NotImplementedError("attention masks with holes are not supported")
                 valid[b] = slice(int(idx[0]), int(idx[0]) + lens[b]) if lens[b] else slice(0, 0)
         llm = self.llm
-        for b in range(len(llm.cache.owned)):
-            llm.cache.release(b)
+        llm.release_all()
         if B == 1:
             hid = llm.prefill_hidden(inputs_embeds[0, valid[0]], 0, 0)
         else:  # one packed pass over all rows of the batch
@@ -310,7 +351,13 @@ class LlavaLlamaModel:
         for b in range(B):
             logits[b, valid[b]] = lg[o:o + lens[b]]
             o += lens[b]
-        return CausalLMOutputWithPast(logits=logits)
+        handle = past_key_values
+        if handle is None and use_cache and B == 1 and type(llm).__name__ != "TPLlamaDecoder":
+            handle = PagedKVCacheHandle()
+        if handle is not None:
+            handle.update(llm, inputs_embeds[0, valid[0]].to(self.dtype), lens[0])
+            handle.last_reused = 0
+        return CausalLMOutputWithPast(logits=logits, past_key_values=handle)
 
     __call__ = forward
 
@@ -334,6 +381,7 @@ class LlavaLlamaModel:
         eos_token_id = generation_kwargs.pop("eos_token_id", self.config.llama.eos_token_id)
         return_logits = bool(generation_kwargs.pop("output_logits", False))
         use_graph = bool(generation_kwargs.pop("use_cuda_graph", True))
+        handle = generation_kwargs.pop("past_key_values", None)
         # do_sample=True -> HF's TemperatureLogitsWarper + TopPLogitsWarper + multinomial, here one kernel per token
         # (eval_spatial.py:231-236 passes do_sample = temperature > 0, so temperature 0 stays greedy)
         sampling = None
@@ -345,6 +393,8 @@ class LlavaLlamaModel:
             raise NotImplementedError("beam search is implemented for do_sample=False without output_logits (the eval scripts' mode)")
         if generation_kwargs:
             raise TypeError(f"unsupported generation kwargs: {sorted(generation_kwargs)}")
+        if handle is not None:  # HF semantics: input_ids is the WHOLE sequence; the cached prefix is found by comparing input rows
+            self._check_handle(handle, input_ids.shape[0], num_beams)
 
         packed = None
         if images is not None:
@@ -378,12 +428,20 @@ class LlavaLlamaModel:
         elif B == 1:
             n = lens[0]
             emb = packed if packed is not None else (inputs_embeds[0, inputs_embeds.shape[1] - n:] if left else inputs_embeds[0, :n])
+            reuse = 0
+            if handle is not None:
+                reuse = reusable_prefix(emb, handle.rows, handle.length, handle.is_live_for(self.llm))
             r = self.llm.generate_from_embeds(emb, int(max_new_tokens), eos_token_ids=eos_token_id, stopping_fn=stop_fn,
-                                              use_graph=use_graph, return_logits=return_logits, sampling=sampling)
+                                              use_graph=use_graph, return_logits=return_logits, sampling=sampling, prefix_len=reuse)
             if return_logits:
                 r, lg = r
                 all_logits.append(lg)
             outs.append(r)
+            if handle is not None and r.numel():
+                # the handle now describes prompt + answer; the KV of the last answer token is not final (cached_length)
+                rows = torch.cat([emb.to(self.dtype), self.llm.embed_tokens(r)], 0)
+                handle.update(self.llm, rows, LlamaDecoder.cached_length(n, r.numel()))
+                handle.last_reused = reuse
         else:
             # batch > 1: one packed prefill over all prompts (llava_arch.py:549-611 pads, modeling_llama.py:540-562 unpads
             # again; here the rows were never padded), then per-sequence decode

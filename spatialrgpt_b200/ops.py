@@ -322,6 +322,41 @@ def attention_prefill_varlen(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, 
     return out
 
 
+def attention_prefill_paged_workspace(n_seqs: int, max_q_len: int, max_ctx_len: int, n_heads: int, n_kv_heads: int, device) -> Optional[torch.Tensor]:
+    """fp32 partials of the paged kernel's context split for this shape (None when the shape runs unsplit)."""
+    n = _lib.load().srgpt_attention_prefill_paged_workspace(n_seqs, max_q_len, max_ctx_len, n_heads, n_kv_heads)
+    if n < 0:
+        raise SrgptError(f"attention_prefill_paged: unsupported shape n_seqs={n_seqs} max_q_len={max_q_len} max_ctx_len={max_ctx_len} "
+                         f"heads={n_heads}/{n_kv_heads}")
+    return torch.empty(n // 4, dtype=torch.float32, device=device) if n else None
+
+
+def attention_prefill_paged(q: torch.Tensor, kv_pages: torch.Tensor, page_tables: torch.Tensor, page_size: int, cu_q: torch.Tensor,
+                            start_pos: torch.Tensor, max_q_len: int, max_ctx_len: int, n_heads: int, n_kv_heads: int, head_dim: int,
+                            scale: float, out: Optional[torch.Tensor] = None, split: bool = True) -> torch.Tensor:
+    """New rows over the paged cache of ONE layer (modeling_llama.py:451-456 + 564-566 with q_len < kv_len): rows
+    [cu_q[b], cu_q[b+1]) of q [rows, >= n_heads*head_dim] are sequence b's rows at positions start_pos[b] + i, each attends to
+    positions 0..p through page_tables[b].  The rows' own K/V must already be in the pages.  ``split=False`` runs without the
+    context split (one CTA walks the whole context)."""
+    _need(q, ELEM(), "attention_prefill_paged.q")
+    _need(kv_pages, ELEM(), "attention_prefill_paged.kv_pages")
+    for t, nm in ((page_tables, "page_tables"), (cu_q, "cu_q"), (start_pos, "start_pos")):
+        _need(t, torch.int32, f"attention_prefill_paged.{nm}")
+    n_seqs = cu_q.numel() - 1
+    if page_tables.dim() != 2 or page_tables.shape[0] < n_seqs or page_tables.stride(1) != 1 or start_pos.numel() < n_seqs:
+        raise SrgptError("attention_prefill_paged: page_tables [n_seqs, cap] / start_pos [n_seqs] expected")
+    if out is None:
+        out = torch.empty((q.shape[0], n_heads * head_dim), dtype=ELEM(), device=q.device)
+    ws = attention_prefill_paged_workspace(n_seqs, max_q_len, max_ctx_len, n_heads, n_kv_heads, q.device) if split else None
+    check(_lib.load().srgpt_attention_prefill_paged_bf16(_p(q), _rowmajor2d(q, "q"), _p(out), _rowmajor2d(out, "out"), _p(kv_pages), _p(page_tables),
+                                                         page_tables.stride(0), page_size, n_seqs, _p(cu_q), _p(start_pos), max_q_len, max_ctx_len,
+                                                         n_heads, n_kv_heads, head_dim, scale, _p(ws), 0 if ws is None else ws.numel() * 4, _stream()),
+          "srgpt_attention_prefill_paged_bf16")
+    if ws is not None:
+        _count(2)
+    return out
+
+
 def rope_kv_append_varlen(qkv: torch.Tensor, n_heads: int, n_kv_heads: int, head_dim: int, cos_tab: torch.Tensor, sin_tab: torch.Tensor,
                           start_pos: torch.Tensor, kv_pages: torch.Tensor, page_tables: torch.Tensor, page_size: int,
                           cu_seqlens: torch.Tensor) -> None:
@@ -616,6 +651,35 @@ def llama_prefill_layers(x: torch.Tensor, layer_array, n_layers: int, dims, cos,
                                                       _p(start_pos), _p(page_table), page_size, n_seqs, _p(cu_seqlens), max_seqlen, pt_stride,
                                                       _stream()), "srgpt_llama_prefill_layers_bf16")
     _count(8 * n_layers)
+    return x
+
+
+def llama_prefill_layers_paged(x: torch.Tensor, layer_array, n_layers: int, dims, cos, sin, start_pos, page_tables, page_size: int,
+                               cu_seqlens: torch.Tensor, max_seqlen: int, max_ctx_len: int) -> torch.Tensor:
+    """All decoder layers over new rows x [S, H] in place that CONTINUE cached sequences: chunk b (rows [cu_seqlens[b],
+    cu_seqlens[b+1])) sits at positions start_pos[b].. and attends to everything its sequence has cached (page_tables [n_seqs, cap])."""
+    _need(x, ELEM(), "llama_prefill_layers_paged.x")
+    for t, nm in ((start_pos, "start_pos"), (page_tables, "page_tables"), (cu_seqlens, "cu_seqlens")):
+        _need(t, torch.int32, f"llama_prefill_layers_paged.{nm}")
+    n_seqs = cu_seqlens.numel() - 1
+    if page_tables.dim() != 2 or page_tables.shape[0] < n_seqs or start_pos.numel() < n_seqs or page_tables.stride(1) != 1:
+        raise SrgptError("llama_prefill_layers_paged: page_tables [n_seqs, cap] and start_pos [n_seqs] expected")
+    _ensure_gemm_workspace(x.device)
+    S, H = x.shape
+    nh, nkv, hd, I = dims.num_attention_heads, dims.num_key_value_heads, dims.head_dim, dims.intermediate_size
+    dev = x.device
+    ws_h = torch.empty((S, H), dtype=ELEM(), device=dev)
+    ws_qkv = torch.empty((S, (nh + 2 * nkv) * hd), dtype=ELEM(), device=dev)
+    ws_attn = torch.empty((S, nh * hd), dtype=ELEM(), device=dev)
+    ws_act = torch.empty((S, I), dtype=ELEM(), device=dev)
+    ws_split = attention_prefill_paged_workspace(n_seqs, max_seqlen, max_ctx_len, nh, nkv, dev)
+    import ctypes
+    check(_lib.load().srgpt_llama_prefill_layers_paged_bf16(_p(x), ctypes.cast(layer_array, ctypes.c_void_p), n_layers, _p(ws_h), _p(ws_qkv),
+                                                            _p(ws_attn), _p(ws_act), _p(ws_split), 0 if ws_split is None else ws_split.numel() * 4,
+                                                            S, H, nh, nkv, hd, I, dims.rms_norm_eps, _p(cos), _p(sin), _p(start_pos), _p(page_tables),
+                                                            page_tables.stride(0), page_size, n_seqs, _p(cu_seqlens), max_seqlen, max_ctx_len, _stream()),
+          "srgpt_llama_prefill_layers_paged_bf16")
+    _count((8 + (ws_split is not None)) * n_layers)
     return x
 
 
